@@ -12,6 +12,11 @@ through rb_world_step_host with HOST state buffers (H2D of every body state + D2
 the timed region).  The reference arm is the CPU oracle (`oracle/`, a scalar restatement -- the Rust
 reference cannot be built in this image, see DESIGN.md), built -O3 -march=native on the host it runs on and run
 with the thread count that is fastest for the scene (swept; the sweep is printed).
+
+bench.py runs the library that `__graft_entry__.build()` left in the tree and writes nothing there (the CPU arm's
+host-specific build goes to a temporary directory), so the tree may be read-only.  --dump-outputs DIR writes the body
+poses and velocities the last timed step left, as DIR/<scene>_pose.npy (n x 7) and DIR/<scene>_vel.npy (n x 6), float32:
+the scenes are fixed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -21,6 +26,7 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True   # no __pycache__ in the tree
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
@@ -184,6 +190,8 @@ def main():
                     help="b3d_many_pyramids_80x20 = BASELINE.json configs[1] (headline); b3d_many_pyramids = the reference file's 14x14x10")
     ap.add_argument("--l2", default="flush", choices=["flush", "keep"])
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the body states of each timed scene after its last timed step to DIR/<scene>_{pose,vel}.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":
@@ -192,14 +200,11 @@ def main():
 
     import numpy as np
     import torch
-    import __graft_entry__ as ge
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world_size = int(os.environ.get("WORLD_SIZE", "1"))
     if world_size != args.gpus:
         raise SystemExit(f"--gpus {args.gpus} but WORLD_SIZE={world_size}: launch with torchrun --nproc-per-node {args.gpus}")
-    if rank == 0:
-        ge.build()
     dist = None
     if world_size > 1:
         import torch.distributed as dist
@@ -244,6 +249,14 @@ def main():
         torch.cuda.synchronize()
         return sum(a.elapsed_time(b) for a, b in evs)
 
+    def dump_outputs(name):
+        """The body states as a caller of the timed path receives them (float32 pose n x 7, velocity n x 6)."""
+        if args.dump_outputs and rank == 0:
+            pose, vel = pipe.body_states()
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, f"{name}_pose.npy"), pose)
+            np.save(os.path.join(args.dump_outputs, f"{name}_vel.npy"), vel)
+
     for _ in range(args.warmup):
         one_step()
     torch.cuda.synchronize()
@@ -260,6 +273,7 @@ def main():
         # per-launch-group device times for the roofline (events inside the library, same stream)
         if exchange is not None:
             shard.finish()   # no gather may be in flight while steps run without exchange() in between
+        dump_outputs(args.scene)   # after finish(): rank 0 holds the states of every body
         pipe.enable_profiling(True)
         prof = {"collision_detection_ms": 0.0, "solver_ms": 0.0}
         nprof = min(args.steps, 100)
@@ -349,6 +363,7 @@ def main():
         torch.cuda.synchronize()
         k2 = min(args.steps, 100)
         ms2 = timed_steps(k2)
+        dump_outputs("b3d_many_pyramids")
         c2 = pipe.counters()
         other = {"workload": workload_name("b3d_many_pyramids", 1), "value": k2 / (ms2 / 1000.0), "unit": "steps/s",
                  "ms_per_step": ms2 / k2, "steps": k2, "bodies": c2["num_bodies"] - 1, "manifolds": c2["num_active_manifolds"]}

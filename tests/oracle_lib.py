@@ -1,8 +1,11 @@
 """ctypes wrapper of the CPU oracle (oracle/_build/liborc.so).  TEST INFRASTRUCTURE ONLY:
 imported by tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs."""
+import atexit
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -21,29 +24,17 @@ def build():
 _libs = {}
 
 
-def _cpu_tag():
-    """Hash of this host's CPU feature flags: the -march=native baseline build is only valid where it was built."""
-    import hashlib
-    flags = ""
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("flags"):
-                flags = line
-                break
-    except OSError:
-        pass
-    return hashlib.sha1(flags.encode()).hexdigest()[:10]
-
-
 def lib(fast=False):
     """fast=False: the bit-exact oracle (the parity checker).  fast=True: the CPU-baseline build of the same sources
-    (-O3 -march=native, built on this host; bench.py's cpu_baseline / --impl reference legs only)."""
+    (-O3 -march=native, built by this process into a temporary directory that is removed when it exits: the binary
+    only fits this host, and bench.py must leave the tree untouched; bench.py's cpu_baseline / --impl reference legs)."""
     if fast not in _libs:
         path = LIB_PATH
         if fast:
-            tag = _cpu_tag()
-            path = os.path.join(ORACLE_DIR, "_build", f"liborc_fast_{tag}.so")
-            subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "fast", f"FAST_TAG={tag}"])
+            out = tempfile.mkdtemp(prefix="rapier_b200_oracle_fast_")
+            atexit.register(shutil.rmtree, out, True)
+            path = os.path.join(out, "liborc_fast.so")
+            subprocess.check_call(["make", "-s", "-C", ORACLE_DIR, "fast", f"FAST_DIR={out}"])
         elif not os.path.exists(LIB_PATH):
             build()
         L = C.CDLL(path)

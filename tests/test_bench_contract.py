@@ -1,8 +1,12 @@
-"""bench.py's reference arm runs on the CPU, so its JSON contract can be checked without a GPU."""
+"""bench.py's reference arm runs on the CPU, so its JSON contract can be checked without a GPU; the GPU arm's
+--dump-outputs is checked on the GPU."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -28,3 +32,24 @@ def test_reference_arm_other_ranks_exit_quietly():
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "2", "--warmup", "3"],
                        capture_output=True, text=True, timeout=600, cwd=ROOT, env=env)
     assert r.returncode == 0 and not [l for l in r.stdout.splitlines() if l.startswith("{")]
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_are_the_states_after_the_last_timed_step(built, tmp_path):
+    """--dump-outputs writes the body states each timed scene holds after warm-up + --steps timed steps, bit for bit
+    what a PhysicsWorld stepped as many times returns."""
+    from rapier_b200 import scenes
+    from rapier_b200.world import PhysicsWorld
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--gpus", "1", "--steps", "4", "--warmup", "3",
+                        "--cpu-seconds", "0.1", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    lines = [l for l in r.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 4
+    for name, scene in (("b3d_many_pyramids_80x20", scenes.pyramids(8, 10, 20)), ("b3d_many_pyramids", scenes.pyramids(14, 14, 10))):
+        w = PhysicsWorld(scene)
+        for _ in range(3 + 4):
+            w.step()
+        for part, want in zip(("pose", "vel"), w.body_states()):
+            got = np.load(tmp_path / f"{name}_{part}.npy")
+            assert got.dtype == np.float32 and got.shape == want.shape, (name, part, got.dtype, got.shape)
+            assert (got.view(np.uint32) == want.view(np.uint32)).all(), (name, part)
